@@ -13,8 +13,9 @@ lm_head and the KV cache are NOT part of the step (they are not on the path this
 `config`.  As `llama.py --include_sparse` always runs (llama.py:301-306), sparse layers use the hybrid symbol with
 topX=10 dense rows that are zero (a checkpoint without them, llama.py:182).
 
-  value  : tokens/s, device-timed, inputs resident in HBM, one CUDA-graph replay per step; --steps K steps per timed block,
-           5 blocks, the MEDIAN block is reported (ms_per_step = median block / K; all block times are in `blocks_ms`).
+  value  : tokens/s, device-timed, inputs resident in HBM, one CUDA-graph replay per step; --steps K timed steps in all, in
+           --blocks (5) blocks of near-equal size, the MEDIAN per-step time of the blocks is reported (ms_per_step; block
+           times in `blocks_ms`, their step counts in `block_steps`).  --dump-outputs DIR writes the last timed step's outputs.
   lut_fp16: the same measurement with the fp16 pair-table mode of the kernel (quant_cuda.set_lut_mode("fp16"), north_star's
            "per-channel fp16 LUT"); the headline `value` always uses the exact fp32 codebook.  `--lut fp16` makes it the only run.
   parity_check: outside the timed region, one sampled layer group per rank against the fp64 CPU oracle on the same buffers.
@@ -118,10 +119,12 @@ def build_model(cfg, dev, rank, world, seed=0):
     return layers, nbytes, nlaunch
 
 
-def make_step(layers, world, peer=None):
+def make_step(layers, world, peer=None, keep=None):
     """Returns (step, run_layer).  step: x [hidden] -> x' [hidden], the 7 matvecs per decoder layer in model order (see module
     docstring).  run_layer(L, x) runs ONE decoder layer the same way and returns [(name, input, full-length output)] for the 7
-    matvecs - what parity_check compares with the oracle (at N > 1: after the exchange, i.e. the vectors the next matvec reads)."""
+    matvecs - what parity_check compares with the oracle (at N > 1: after the exchange, i.e. the vectors the next matvec reads).
+    keep: a list that step() refills with run_layer's result for every layer, so that the 7 x layers output tensors of its last
+    call (in a CUDA graph: of its last replay) stay readable."""
     QKV, GU = ("q_proj", "k_proj", "v_proj"), ("gate_proj", "up_proj")
     if world == 1:
         def run_layer(L, x):
@@ -178,8 +181,13 @@ def make_step(layers, world, peer=None):
             return [("q_proj", x, q), ("k_proj", x, k), ("v_proj", x, v), ("o_proj", v, o), ("gate_proj", o, g), ("up_proj", o, u), ("down_proj", g, d)]
 
     def step(x):
+        if keep is not None:
+            keep.clear()
         for L in layers:
-            x = run_layer(L, x)[-1][2]
+            outs = run_layer(L, x)
+            if keep is not None:
+                keep.append(outs)
+            x = outs[-1][2]
         return x.clone() if world > 1 else x
     return step, run_layer
 
@@ -385,7 +393,15 @@ def main():
     ap.add_argument("--no-fuse", action="store_true", help="one launch per QuantLinearLUT (no q/k/v and gate/up sibling stacking)")
     ap.add_argument("--lut", default="both", choices=["both", "exact", "fp16"],
                     help="codebook precision: exact = fp32 as stored (headline), fp16 = pair tables; both = headline exact + a lut_fp16 object")
-    ap.add_argument("--blocks", type=int, default=5, help="timed blocks of --steps steps each; the median block is reported")
+    ap.add_argument("--blocks", type=int, default=5,
+                    help="the --steps timed steps are split into this many blocks (at most --steps) of near-equal size; the median "
+                         "per-step time of the blocks is reported")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (float32): step_output "
+                         "[hidden] and, with one launch per (stacked) matvec, every matvec's full-length output as <matvec name>.npy "
+                         "[layers, out_features] (an evenly spaced subset of the layers if all of them would exceed 64 MB).  The inputs "
+                         "are seeded; the default summation order is not, so two runs differ by fp16 roundings that grow along the "
+                         "chain (LLaMA-7B w4-s45, two runs on one B200: up to 5e-4 of max|y| in layer 0, 4e-3 in layer 31)")
     ap.add_argument("--per-shape", action="store_true",
                     help="also time each of the step's launch types on its own (one CUDA graph of `layers` launches over every layer's "
                          "distinct weights, CUDA events) and add a per_shape object: us per launch, GB/s and roofline fraction per type")
@@ -394,6 +410,7 @@ def main():
     if args.layers:
         cfg["layers"] = args.layers
     assert args.warmup >= 3, "timing rules: at least 3 warm-up steps"
+    assert args.steps >= 1 and args.blocks >= 1, "--steps and --blocks must be at least 1"
 
     if args.impl == "reference":
         run_reference_arm(args, cfg)
@@ -439,9 +456,10 @@ def main():
     if world > 1 and use_seq:
         from squeezellm_b200.sharding import PeerArena
         seq_peer = PeerArena(rank, world, dev)
+    keep = [] if args.dump_outputs and not use_seq else None  # the sequence kernel hands out the step's output only
     if world > 1:
         import torch.distributed as dist
-        step_nccl, run_layer_nccl = make_step(layers, world)
+        step_nccl, run_layer_nccl = make_step(layers, world, keep=keep)
         run_layer = run_layer_nccl
         step, exchange_used = step_nccl, "nccl all-reduce per launch"
         if use_seq:
@@ -452,7 +470,7 @@ def main():
             try:
                 from squeezellm_b200.sharding import PeerExchange
                 peer = PeerExchange(rank, world, dev)
-                step_p2p, run_layer_p2p = make_step(layers, world, peer)
+                step_p2p, run_layer_p2p = make_step(layers, world, peer, keep=keep)
                 xs = torch.randn(cfg["hidden"], device=dev, generator=torch.Generator(device=dev).manual_seed(7)).half()
                 a, b = step_p2p(xs).float(), step_nccl(xs).float()
                 torch.cuda.synchronize()
@@ -471,7 +489,7 @@ def main():
             elif why or rank == 0:
                 print(f"[bench] rank {rank}: p2p exchange not used ({why or 'another rank declined'}); falling back to NCCL", file=sys.stderr)
     else:
-        step, run_layer = make_step(layers, world)
+        step, run_layer = make_step(layers, world, keep=keep)
     x0 = torch.randn(cfg["hidden"], device=dev, generator=torch.Generator(device=dev).manual_seed(99)).half()  # same on every rank
 
     def barrier():
@@ -482,12 +500,13 @@ def main():
 
     from squeezellm_b200.quant import quant_cuda
     from squeezellm_b200.runtime import GraphedDecodeStep
-    xh = torch.randn(cfg["hidden"]).half().pin_memory()
+    xh = torch.randn(cfg["hidden"], generator=torch.Generator().manual_seed(98)).half().pin_memory()
     sampler = ClockSampler(torch.cuda.current_device() if "CUDA_VISIBLE_DEVICES" not in os.environ else local)
 
-    def measure(lut_mode, sample_clocks):
+    def measure(lut_mode, sample_clocks, dump=False):
         """One full measurement (device-resident blocks, then end to end from host memory) with the given codebook mode.
-        The mode is baked into the graph at capture time (the kernel variant is chosen per launch)."""
+        The mode is baked into the graph at capture time (the kernel variant is chosen per launch).
+        dump: also return the outputs of the last timed step (name -> float32 host tensor)."""
         quant_cuda.set_lut_mode(lut_mode)
         graphed = True
         seq = None
@@ -506,10 +525,7 @@ def main():
             torch.cuda.synchronize()
 
         def one_step():
-            if graphed:
-                runner.replay()
-            else:
-                step(x0)
+            return runner.replay() if graphed else step(x0)
 
         for _ in range(args.warmup):
             one_step()
@@ -522,15 +538,22 @@ def main():
             barrier()
         if sample_clocks and rank == 0:
             sampler.start()
-        evs = [torch.cuda.Event(enable_timing=True) for _ in range(args.blocks + 1)]
+        nblocks = min(args.blocks, args.steps)
+        sizes = [args.steps // nblocks + (b < args.steps % nblocks) for b in range(nblocks)]  # args.steps timed steps in all
+        evs = [torch.cuda.Event(enable_timing=True) for _ in range(nblocks + 1)]
         evs[0].record()
-        for b in range(args.blocks):
-            for _ in range(args.steps):
-                one_step()
+        for b in range(nblocks):
+            for _ in range(sizes[b]):
+                y = one_step()
             evs[b + 1].record()
         barrier()
-        blocks = [evs[b].elapsed_time(evs[b + 1]) for b in range(args.blocks)]
+        blocks = [evs[b].elapsed_time(evs[b + 1]) for b in range(nblocks)]
         clocks = sampler.stop() if (sample_clocks and rank == 0) else None
+        outputs = None
+        if dump:  # read before the end-to-end run below overwrites the graph's buffers
+            outputs = {"step_output": y.float().cpu()}
+            for j, name in enumerate([o[0] for o in keep[0]] if keep else []):
+                outputs[name] = torch.stack([outs[j][2].reshape(-1) for outs in keep]).float().cpu()
         # end to end from host memory through the public API
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         if graphed:
@@ -557,7 +580,7 @@ def main():
             t = torch.tensor(blocks + [e2e_ms], device=dev, dtype=torch.float64)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)  # every block: max over ranks
             blocks, e2e_ms = t.tolist()[:-1], t.tolist()[-1]
-        ms = statistics.median(blocks)
+        ms_step = statistics.median([ms / n for ms, n in zip(blocks, sizes)])
         quant_cuda.set_lut_mode("exact")
         seq_timeout = False
         if seq is not None:
@@ -566,8 +589,8 @@ def main():
                 print(f"[bench] rank {rank}: the sequence kernel's error word is set after the timed region - THIS RUN'S NUMBERS ARE VOID", file=sys.stderr)
             del runner, seq
             torch.cuda.empty_cache()
-        return {"seq_timeout": seq_timeout, "warm_timeout": warm_timeout, "ms_step": ms / args.steps, "e2e_ms_step": e2e_ms / args.steps, "blocks_ms": [round(b, 4) for b in blocks],
-                "graphed": graphed, "clocks": clocks}
+        return {"seq_timeout": seq_timeout, "warm_timeout": warm_timeout, "ms_step": ms_step, "e2e_ms_step": e2e_ms / args.steps, "blocks_ms": [round(b, 4) for b in blocks],
+                "block_steps": sizes, "graphed": graphed, "clocks": clocks, "outputs": outputs}
 
     def per_shape(lut_mode):
         """us per launch for each launch type of the step: a graph with one launch per decoder layer (every layer's own weights, LUT
@@ -619,7 +642,7 @@ def main():
     shapes = None
     if args.per_shape and world == 1:
         shapes = {"exact": per_shape("exact"), "fp16": per_shape("fp16")}
-    main_run = measure(head_mode, True)
+    main_run = measure(head_mode, True, dump=bool(args.dump_outputs))
     extra_run = measure("fp16", False) if args.lut == "both" else None
 
     # ---- parity: one sampled layer group per rank against the fp64 oracle on the same buffers (outside every timed region) ----------
@@ -682,8 +705,9 @@ def main():
                    "parallelism": "single GPU" if world == 1 else f"column-sharded x{world}, {nlaunch} launches per step", "exchange": exchange_used,
                    "launch": ("one CUDA-graph replay per step" if graphed else "eager launches (graph capture unavailable)") +
                              (": ONE persistent kernel runs all matvecs of the token (runtime.DecodeSequence)" if use_seq else ": one PDL-chained launch per (stacked) matvec"),
-                   "lut": head_mode, "timing": f"median of {args.blocks} blocks of {args.steps} steps", "layers_timed": cfg["layers"]},
-        "blocks_ms": main_run["blocks_ms"],
+                   "lut": head_mode, "timing": f"{args.steps} timed steps in {len(main_run['block_steps'])} blocks, median per-step time of the blocks",
+                   "layers_timed": cfg["layers"]},
+        "blocks_ms": main_run["blocks_ms"], "block_steps": main_run["block_steps"],
         "e2e": {"value": e2e_tok_s, "unit": "tokens/s", "h2d_bytes_per_step": cfg["hidden"] * 2, "d2h_bytes_per_step": cfg["hidden"] * 2,
                 "api": ("squeezellm_b200.runtime.GraphedDecodeStep over runtime.DecodeSequence (QuantLinearLUT modules)" if use_seq else
                         "squeezellm_b200.runtime.GraphedDecodeStep over QuantLinearLUT.forward") if graphed else "QuantLinearLUT.forward eager"},
@@ -713,8 +737,29 @@ def main():
                                "fused_lookup_gemv_port_tokens_per_s": 1.0 / (min(fused) * cfg["layers"]), "fused_port_threads": thr,
                                "matmul_only_on_predequantized_fp16_tokens_per_s": 1.0 / (min(cpu_layer_sample.matmul_only) * cfg["layers"]),
                                "host_cpus": os.cpu_count()}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, main_run["outputs"])
     print(json.dumps(out), flush=True)
     leave(world)
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, outputs):
+    """outputs: name -> float32 tensor on the host; [layers, N] arrays keep an evenly spaced subset of their rows (first and last
+    layer included) if all of them would exceed DUMP_BYTES."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    per_layer = sum(v[0].numel() * 4 for k, v in outputs.items() if k != "step_output")
+    nlayers = max((len(v) for k, v in outputs.items() if k != "step_output"), default=0)
+    nrows = min(nlayers, (DUMP_BYTES - outputs["step_output"].numel() * 4) // per_layer) if per_layer else 0
+    rows = np.unique(np.linspace(0, nlayers - 1, nrows).round().astype(np.int64))
+    for name, v in outputs.items():
+        a = v.numpy().astype(np.float32)
+        if name != "step_output":
+            a = a[rows]
+        np.save(os.path.join(path, f"{name}.npy"), a)
 
 
 def parity_check(layers, run_layer, cfg, rank, world, dev, quant_cuda):

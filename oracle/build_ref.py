@@ -13,8 +13,9 @@ Recipe for `oracle/_ref/` (git-ignored, travels to the GPU box with gpurun):
     can live in the same process as our own `quant_cuda`;
   * only the resulting `.so` is written to oracle/_ref/.
 
-The product (squeezellm_b200/, bench.py's own arm) never imports this.  Users: tests/ (parity vs the
-reference kernel on the B200), tests/golden/make_golden_gpu.py, oracle/ref_gpu_timing.py.
+The product (squeezellm_b200/, bench.py's own arm) never imports this, nor do the tests.  Users:
+tests/golden/make_golden_gpu.py and tests/golden/make_golden_parity.py (the reference outputs the tests compare
+against), oracle/ref_gpu_timing.py.
 """
 import glob
 import os

@@ -2,10 +2,11 @@
 declares, argument validation answers without touching a GPU, and the `quant_cuda` module carries the
 reference's 12 names (squeezellm/quant_cuda.cpp:258-269)."""
 import ctypes
+import os
 
 import pytest
 
-from util import Args, header_symbols, load_lib
+from util import GOLDEN, Args, buffer_signature, header_symbols, load_lib
 
 REFERENCE_SYMBOLS = [
     "vecquant3matmul_nuq_perchannel", "vecquant4matmul_nuq_perchannel",
@@ -106,22 +107,21 @@ def test_exchange_descriptor_validation_without_gpu(change, frag):
 
 def test_reference_quant_py_imports_against_our_extension():
     """Option A of INTEGRATION.md: the reference's own squeezellm/quant.py, unmodified, imports `quant_cuda` by name and finds every
-    symbol it calls in OUR extension (except the *_balanced_* ones, which the reference's extension does not define either).
-    Needs the reference checkout; skipped where it is absent (e.g. on the GPU box)."""
-    import importlib.util
-    import os
-    import re
-    ref = "/root/reference/squeezellm/quant.py"
-    if not os.path.exists(ref):
-        pytest.skip("reference checkout not present")
-    import squeezellm_b200.quant as ours            # puts the in-tree extension directory on sys.path, imports quant_cuda
-    spec = importlib.util.spec_from_file_location("reference_quant", ref)
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)                     # runs `import quant_cuda` (quant.py:5)
-    assert mod.quant_cuda is ours.quant_cuda
-    called = set(re.findall(r"quant_cuda\.(\w+)", open(ref).read()))
-    missing = {n for n in called if not hasattr(mod.quant_cuda, n)}
+    symbol it calls in OUR extension (except the *_balanced_* ones, which the reference's extension does not define either), and its
+    QuantLinearLUT registers the same buffers as ours.  What quant.py calls and registers is recorded in
+    tests/golden/reference_quant_api.json (tests/golden/make_golden_reference_api.py)."""
+    import json
+    import squeezellm_b200.quant as ours            # registers the in-tree extension as top-level module `quant_cuda`
+    import quant_cuda                                # what quant.py:5 runs
+    assert quant_cuda is ours.quant_cuda
+    with open(os.path.join(GOLDEN, "reference_quant_api.json")) as f:
+        rec = json.load(f)
+    called = set(rec["quant_cuda_calls"])
+    missing = {n for n in called if not hasattr(quant_cuda, n)}
     assert len(called - missing) == 12
     assert missing and all("balanced" in n for n in missing), missing
-    m = mod.QuantLinearLUT(4, 128, 128, False, include_sparse=True, numvals=5, topX=10)   # the reference's module over our extension
-    assert set(m.state_dict()) == set(ours.QuantLinearLUT(4, 128, 128, False, include_sparse=True, numvals=5, topX=10).state_dict())
+    assert rec["modules"]
+    for mod in rec["modules"]:
+        bits, K, N, bias, sparse, numvals, topx = mod["args"]
+        m = ours.QuantLinearLUT(bits, K, N, bias, include_sparse=sparse, numvals=numvals, topX=topx)
+        assert {k: buffer_signature(v) for k, v in m.state_dict().items()} == mod["buffers"], mod["args"]

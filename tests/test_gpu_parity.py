@@ -1,6 +1,7 @@
 """GPU parity tests (run on the B200 with `-m gpu`): our CUDA path, called through the C ABI (ctypes on
 libsqllm_b200.so) and through the `quant_cuda` module, against the CPU oracle on the same seeded inputs, and
-against the reference's own kernels (oracle/_ref) when that build travelled with the tree."""
+against the outputs of the reference's own kernels for the same inputs (tests/golden/refparity_*.npz, written on a
+B200 by tests/golden/make_golden_parity.py)."""
 import ctypes
 import os
 
@@ -8,7 +9,7 @@ import numpy as np
 import pytest
 import torch
 
-from util import Args, REL_TOL, TIGHT_TOL, ROOT, load_lib, orc, rel_err, to_torch
+from util import GOLDEN, Args, REL_TOL, TIGHT_TOL, load_lib, orc, rel_err, to_torch
 
 pytestmark = pytest.mark.gpu
 
@@ -40,15 +41,43 @@ SHAPES = [  # (bits, K, N, sparsity, topX, nonzero_full_rows, skew)
     (3, 11008, 64, 0.01, 4, True, False),       # one strip, every CTA inside it: 147 mailbox rows for one owner
 ]
 IDS = [f"w{b}-{k}x{n}-s{int(s*1e4)}-t{t}{'-nz' if z else ''}{'-skew' if sk else ''}" for b, k, n, s, t, z, sk in SHAPES]
+BATCHED_SHAPES = [s for s in SHAPES if s[1] <= 512] + [(4, 4096, 4096, 0.0045, 10, True, False), (3, 11008, 4096, 0.0045, 10, True, True)]
+BATCHES = [2, 5, 16, 64]
 
 
-def _ref_module():
-    import sys
-    sys.path.insert(0, os.path.join(ROOT, "oracle"))
-    import build_ref
-    if not build_ref.have_ref_so():
-        return None
-    return build_ref.load()
+def batched_id(s):
+    return f"w{s[0]}-{s[1]}x{s[2]}-t{s[4]}"
+
+
+def _layer(shape, seed):
+    bits, K, N, sp, topx, nz, skew = shape
+    L = orc.make_layer(bits, K, N, sparsity=sp, topX=topx, seed=seed, skew=skew, nonzero_full_rows=nz)
+    if topx and sp == 0:
+        L["full_rows"] = L["full_row_indices"] = None
+    return L
+
+
+def matvec_case(shape):
+    """Layer and x of test_matvec_module_vs_reference_kernel."""
+    return _layer(shape, shape[1] + shape[2] + shape[0]), orc.make_vec(shape[1], seed=2)
+
+
+def batched_case(shape, batch):
+    """Layer and x [batch, K] of test_batched_symbols_vs_oracle_and_reference."""
+    return _layer(shape, 3), orc.make_vec(shape[1], batch=batch, seed=3)
+
+
+def fingerprint(L, x):
+    """Sums of every input array: stored reference outputs are only valid for the inputs they were computed from."""
+    keys = ("qweight", "lookup_table", "rows", "cols", "vals", "full_rows", "full_row_indices")
+    return np.array([np.asarray(a, dtype=np.float64).sum() for a in [L[k] for k in keys if L[k] is not None] + [x]])
+
+
+def vs_reference(got, stored, key, L, x):
+    """rel_err of our output against the reference kernel's, at the output positions stored for case `key`."""
+    assert f"{key}.ref" in stored.files, f"no stored reference output for {key}: run tests/golden/make_golden_parity.py"
+    assert np.allclose(stored[f"{key}.fingerprint"], fingerprint(L, x), rtol=1e-9, atol=0), f"{key}: inputs differ from the stored ones"
+    return rel_err(np.asarray(got).reshape(-1)[stored[f"{key}.idx"]], stored[f"{key}.ref"])
 
 
 @pytest.fixture(scope="module")
@@ -64,7 +93,8 @@ def qc():
 
 @pytest.fixture(scope="module")
 def ref():
-    return _ref_module()
+    """Outputs of the reference's kernels: {"matvec": npz, "batched": npz}."""
+    return {k: np.load(os.path.join(GOLDEN, f"refparity_{k}.npz")) for k in ("matvec", "batched")}
 
 
 def _abi_call(lib, T, x, mul, batch=1):
@@ -119,45 +149,28 @@ def test_matvec_c_abi_vs_oracle(lib, shape):
 
 @pytest.mark.parametrize("shape", SHAPES, ids=IDS)
 def test_matvec_module_vs_reference_kernel(qc, ref, shape):
-    """Identical packed weights and inputs through the reference's own kernels on this GPU (north_star's parity statement)."""
-    if ref is None:
-        pytest.skip("oracle/_ref not built (needs /root/reference at build time)")
-    bits, K, N, sp, topx, nz, skew = shape
-    if K % 128 or N % 128:
-        pytest.skip("reference kernels read out of bounds unless in % 128 == 0 and out % 128 == 0 (SURVEY 2.1)")
-    L = orc.make_layer(bits, K, N, sparsity=sp, topX=topx, seed=K + N + bits, skew=skew, nonzero_full_rows=nz)
-    if topx and sp == 0:
-        L["full_rows"] = L["full_row_indices"] = None
-    x = torch.from_numpy(orc.make_vec(K, seed=2)).cuda().reshape(-1)
+    """Identical packed weights and inputs through the reference's own kernels on a B200 (north_star's parity statement; shapes
+    that are not multiples of 128 ran zero-padded, see make_golden_parity.py)."""
+    L, x = matvec_case(shape)
     T = to_torch(L)
-    ours, theirs = torch.zeros(N, device="cuda"), torch.zeros(N, device="cuda")
-    _module_call(qc, T, x, ours, batched=False)
-    _module_call(ref, T, x, theirs, batched=False)
+    ours = torch.zeros(shape[2], device="cuda")
+    _module_call(qc, T, torch.from_numpy(x).cuda().reshape(-1), ours, batched=False)
     torch.cuda.synchronize()
-    assert rel_err(ours.cpu().numpy(), theirs.cpu().numpy()) < REL_TOL
+    assert vs_reference(ours.cpu().numpy(), ref["matvec"], IDS[SHAPES.index(shape)], L, x) < REL_TOL
 
 
-@pytest.mark.parametrize("shape", [s for s in SHAPES if s[1] <= 512] + [(4, 4096, 4096, 0.0045, 10, True, False), (3, 11008, 4096, 0.0045, 10, True, True)],
-                         ids=lambda s: f"w{s[0]}-{s[1]}x{s[2]}-t{s[4]}")
-@pytest.mark.parametrize("batch", [2, 5, 16, 64])
+@pytest.mark.parametrize("shape", BATCHED_SHAPES, ids=batched_id)
+@pytest.mark.parametrize("batch", BATCHES)
 def test_batched_symbols_vs_oracle_and_reference(qc, ref, shape, batch):
-    bits, K, N, sp, topx, nz, skew = shape
-    L = orc.make_layer(bits, K, N, sparsity=sp, topX=topx, seed=3, skew=skew, nonzero_full_rows=nz)
-    if topx and sp == 0:
-        L["full_rows"] = L["full_row_indices"] = None
-    x = orc.make_vec(K, batch=batch, seed=3)
+    L, x = batched_case(shape, batch)
     T = to_torch(L)
     xs = torch.from_numpy(x).cuda()
-    ours = torch.zeros((batch, N), device="cuda")
+    ours = torch.zeros((batch, shape[2]), device="cuda")
     _module_call(qc, T, xs, ours, batched=True)
     torch.cuda.synchronize()
     want = orc.forward_f64(L, x)
     assert rel_err(ours.cpu().numpy(), want) < TIGHT_TOL
-    if ref is not None and K % 128 == 0 and N % 128 == 0:
-        theirs = torch.zeros((batch, N), device="cuda")
-        _module_call(ref, T, xs, theirs, batched=True)
-        torch.cuda.synchronize()
-        assert rel_err(ours.cpu().numpy(), theirs.cpu().numpy()) < REL_TOL
+    assert vs_reference(ours.cpu().numpy(), ref["batched"], f"{batched_id(shape)}-b{batch}", L, x) < REL_TOL
 
 
 @pytest.mark.parametrize("shape", SHAPES, ids=IDS)

@@ -36,6 +36,11 @@ def golden_files(prefix):
     return sorted(glob.glob(os.path.join(GOLDEN, prefix + "*.npz")))
 
 
+def buffer_signature(t):
+    """'int32[16, 128]': dtype and shape of a state_dict tensor, as tests/golden/reference_quant_api.json records them."""
+    return f"{str(t.dtype).replace('torch.', '')}{list(t.shape)}"
+
+
 def header_symbols():
     txt = open(HEADER).read()
     txt = re.sub(r"/\*.*?\*/", "", txt, flags=re.S)
