@@ -117,7 +117,10 @@ int sqllm_workspace_error(const void *workspace, void *stream);
  * from an fp16 or fp32 x, in ONE launch: replaces torch.zeros (quant.py:218), x.float() (:223,267),
  * the 1-3 reference launches and y.to(dtype) (:311).  Summation order: see sqllm_set_deterministic.
  * x_is_half / y_is_half select the element type of x / y.  bias may be NULL.  x, y and bias must be 16-byte aligned;
- * out_features <= 262144 and topX <= 128 on this path.  args->vec / args->mul / args->batch are ignored. */
+ * out_features <= SQLLM_MAX_N_FUSED and topX <= SQLLM_MAX_TOPX_FUSED on this path (and on the sequence and exchange paths);
+ * sqllm_lutgemv has neither limit.  args->vec / args->mul / args->batch are ignored. */
+#define SQLLM_MAX_TOPX_FUSED 128
+#define SQLLM_MAX_N_FUSED 262144
 int sqllm_lutgemv_fused(const sqllm_lutgemv_args *args,
                         const void *x, int x_is_half, void *y, int y_is_half, const float *bias,
                         void *workspace, size_t workspace_bytes, void *stream);

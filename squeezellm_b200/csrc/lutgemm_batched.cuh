@@ -208,17 +208,19 @@ __global__ void csr_batched_kernel(const int *__restrict__ rows, const int *__re
 }
 
 // topX dense rows for a batch: mul[b][fri[j]] += sum_k full_rows[k][j] * x[b][k].  One CTA per batch row; thread = (k-slice, dense row j):
-// 256 / topX slices of K walk their part with four independent fp32 chains, the slices' sums are added in fixed order through shared
+// 256 / w slices of K walk their part with four independent fp32 chains, the slices' sums are added in fixed order through shared
 // memory (deterministic), one atomicAdd per (b, j).  (First build: one thread per (b, j) walking all K terms in fp64 - 0.37 ms of pure
 // latency whatever the batch, 3x SLOWER than the reference's kernels at batch 16: profiles/r02_batched_vs_reference_kernel.jsonl.)
-__global__ void dense_rows_batched_kernel(const float *__restrict__ full_rows, const int *__restrict__ fri, int topX,
+// Rows go in blocks of w <= 64 (grid.y = ceil(topX / w)), so every row has at least 256 / 64 = 4 k-slices: a layer with hundreds of dense
+// rows keeps its fp32 chains K / 16 long instead of K / 4.  The rows of the last block past topX idle.
+__global__ void dense_rows_batched_kernel(const float *__restrict__ full_rows, const int *__restrict__ fri, int topX, int w,
                                           const float *__restrict__ x, float *__restrict__ mul, int K, int N, int B) {
     __shared__ float part[256];
-    const int b = blockIdx.x, nsl = blockDim.x / topX;
-    const int j = threadIdx.x % topX, sl = threadIdx.x / topX;
+    const int b = blockIdx.x, nsl = blockDim.x / w;
+    const int jl = threadIdx.x % w, j = blockIdx.y * w + jl, sl = threadIdx.x / w;
     const float *xb = x + (size_t)b * K;
     float a0 = 0.f, a1 = 0.f, a2 = 0.f, a3 = 0.f;
-    const int per = (K + nsl - 1) / nsl, k0 = sl * per, k1 = min(K, k0 + per);
+    const int per = (K + nsl - 1) / nsl, k0 = sl * per, k1 = j < topX ? min(K, k0 + per) : k0;
     int k = k0;
     for (; k + 3 < k1; k += 4) {
         a0 = fmaf(__ldg(full_rows + (size_t)k * topX + j), __ldg(xb + k), a0);
@@ -229,9 +231,9 @@ __global__ void dense_rows_batched_kernel(const float *__restrict__ full_rows, c
     for (; k < k1; ++k) a0 = fmaf(__ldg(full_rows + (size_t)k * topX + j), __ldg(xb + k), a0);
     part[threadIdx.x] = (a0 + a1) + (a2 + a3);
     __syncthreads();
-    if (sl == 0) {
+    if (sl == 0 && j < topX) {
         float t = 0.f;
-        for (int i = 0; i < nsl; ++i) t += part[i * topX + j];
+        for (int i = 0; i < nsl; ++i) t += part[i * w + jl];
         const int c = __ldg(fri + j);
         if (c >= 0 && c < N) atomicAdd(mul + (size_t)b * N + c, t);
     }

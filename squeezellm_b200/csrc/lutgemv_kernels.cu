@@ -74,10 +74,10 @@ constexpr int STRIP = 64;                 // output columns per strip (16 lanes 
 constexpr int SU = 2 * NW;                // units per pipeline stage (one pair per consumer warp)
 constexpr int CSR_CH = 1024;              // CSR elements staged per chunk
 constexpr int SROWS_LD = 68;              // padded row-pointer slice per segment (65 used)
-constexpr int MAX_TOPX_FUSED = 128;
+constexpr int MAX_TOPX_FUSED = SQLLM_MAX_TOPX_FUSED;
 constexpr int HYB_R = 11;                 // dense rows: k-rows per lane slot requested before the dependency wait
 constexpr int MAX_STRIPS = 16320;         // per-strip tickets in the workspace header (out_features <= 1,044,480)
-constexpr int MAX_N_FUSED = 262144;        // fused path: the scratch accumulator lives at a fixed place in the workspace
+constexpr int MAX_N_FUSED = SQLLM_MAX_N_FUSED;  // fused path: the scratch accumulator lives at a fixed place in the workspace
 constexpr size_t WS_ACC_OFF = 65536;       // [64 KB, 64 KB + 4*MAX_N_FUSED): fp32 accumulator (zero between launches)
 constexpr int MAX_GRID_V2 = 256;           // v2 runs one CTA per SM
 constexpr size_t WS_HBOX_OFF = WS_ACC_OFF + (size_t)MAX_N_FUSED * 4;       // v2 mailboxes: [MAX_GRID_V2][64] x 8 bytes (partial strip sums)
@@ -2106,9 +2106,8 @@ int launch_batched(const sqllm_lutgemv_args *a, cudaStream_t st) {
         csr_batched_kernel<<<g, blk, 0, st>>>(a->rows, a->cols, a->vals, a->vec, a->mul, K, N, B);
     }
     if (a->full_rows && a->topX > 0) {
-        if (a->topX > 256) return fail(SQLLM_EINVAL, "batched path supports topX <= 256");
-        const int per = 256 / a->topX;
-        dense_rows_batched_kernel<<<B, per * a->topX, 0, st>>>(a->full_rows, a->full_row_indices, a->topX, a->vec, a->mul, K, N, B);
+        const int w = std::min(64, a->topX), per = 256 / w;  // blocks of at most 64 dense rows, any number of them
+        dense_rows_batched_kernel<<<dim3(B, (a->topX + w - 1) / w), per * w, 0, st>>>(a->full_rows, a->full_row_indices, a->topX, w, a->vec, a->mul, K, N, B);
     }
     const cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return fail(SQLLM_ECUDA, "batched launch failed: %s", cudaGetErrorString(e));

@@ -415,4 +415,7 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
           },
           "True if a bounded in-kernel wait of the fused path ever timed out on this stream's workspace (results are then incomplete)");
     m.def("sm_count", []() { return sqllm_device_sm_count(); });
+    // limits of lutgemv_fused, lutgemv_fused_exchange and sequence_create (the 12 accumulate symbols have neither)
+    m.attr("MAX_TOPX_FUSED") = SQLLM_MAX_TOPX_FUSED;
+    m.attr("MAX_N_FUSED") = SQLLM_MAX_N_FUSED;
 }

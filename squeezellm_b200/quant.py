@@ -8,7 +8,8 @@ as the reference, so `llama.py`-style loaders work unchanged.  Differences, all 
   * `forward` (batch-1 branch, reference quant.py:212-312) uses ONE fused launch
     (`quant_cuda.lutgemv_fused`: fp16/fp32 x in, y out in x's dtype, bias + CSR + dense rows fused;
     `quant_cuda.set_deterministic(True)` selects the bit-reproducible summation) instead of
-    zeros + x.float() + 1-3 launches + y.to(dtype).  Set
+    zeros + x.float() + 1-3 launches + y.to(dtype).  Layers past the fused limits (more than
+    quant_cuda.MAX_TOPX_FUSED dense rows or quant_cuda.MAX_N_FUSED output channels) keep the reference sequence.  Set
     `QuantLinearLUT.use_fused = False` to go through the reference's 12 symbols exactly as quant.py does.
   * `balanced=True` raises NotImplementedError up front: the reference dispatches it to
     `vecquant{3,4}matmul_spmv_balanced_nuq_perchannel`, which its extension never defines
@@ -56,6 +57,8 @@ def _load_extension():
 
 
 quant_cuda = _load_extension()
+# limits of the single-launch fused path (the 12 reference symbols have none)
+MAX_TOPX_FUSED, MAX_N_FUSED = quant_cuda.MAX_TOPX_FUSED, quant_cuda.MAX_N_FUSED
 
 
 def round_to_nearest_pole_sim(w, poles):
@@ -164,6 +167,14 @@ class QuantLinearLUT(nn.Module):
             fr, fri = self.full_rows, self.full_row_indices
         return self.rows, self.cols, self.vals, fr, fri
 
+    def fused_ok(self):
+        """True if the single-launch fused path takes this layer: at most MAX_TOPX_FUSED dense rows and at most MAX_N_FUSED
+        output channels.  Past either limit forward() runs the reference sequence, whose symbols have
+        no such limit (a stacked sibling group of three layers with topX = 50 each has 150 dense rows)."""
+        fr = self._sparse_args()[3]
+        topX = fr.shape[1] if fr is not None else 0
+        return topX <= MAX_TOPX_FUSED and self.outfeatures <= MAX_N_FUSED
+
     def forward(self, x):
         if self._sibling_group is not None:
             group, index = self._sibling_group
@@ -172,7 +183,7 @@ class QuantLinearLUT(nn.Module):
         if x.shape[-1] == x.numel():
             outshape = list(x.shape)
             outshape[-1] = self.outfeatures
-            if QuantLinearLUT.use_fused and x.dtype in (torch.float16, torch.float32):
+            if QuantLinearLUT.use_fused and x.dtype in (torch.float16, torch.float32) and self.fused_ok():
                 rows, cols, vals, fr, fri = self._sparse_args()
                 y = quant_cuda.lutgemv_fused(x.contiguous(), self.qweight, self.lookup_table, self.bits,
                                              self.bias, rows, cols, vals, fr, fri)

@@ -99,6 +99,13 @@ class DecodeSequence:
         assert layer.outfeatures % members == 0
         nfull = layer.outfeatures // members * world
         rows, cols, vals, fr, fri = layer._sparse_args()
+        from .quant import MAX_N_FUSED, MAX_TOPX_FUSED
+        topX = fr.shape[1] if fr is not None else 0
+        if topX > MAX_TOPX_FUSED:
+            raise ValueError(f"DecodeSequence: layer has {topX} dense rows; the sequence kernel takes at most MAX_TOPX_FUSED = {MAX_TOPX_FUSED}")
+        if layer.outfeatures > MAX_N_FUSED:
+            raise ValueError(f"DecodeSequence: layer has out_features = {layer.outfeatures}; the sequence kernel takes at most "
+                             f"MAX_N_FUSED = {MAX_N_FUSED}")
         self._items.append((layer.qweight, layer.lookup_table, layer.bits, layer.bias, rows, cols, vals, fr, fri,
                             x.item, x.offset, self.x if x.item < 0 else None, members, nfull))
         self._keep.append(layer)

@@ -2,14 +2,14 @@
 libsqllm_b200.so) and through the `quant_cuda` module, against the CPU oracle on the same seeded inputs, and
 against the outputs of the reference's own kernels for the same inputs (tests/golden/refparity_*.npz, written on a
 B200 by tests/golden/make_golden_parity.py)."""
-import ctypes
 import os
 
 import numpy as np
 import pytest
 import torch
 
-from util import GOLDEN, Args, REL_TOL, TIGHT_TOL, load_lib, orc, rel_err, to_torch
+from util import GOLDEN, REL_TOL, TIGHT_TOL, load_lib, orc, rel_err, to_torch
+from util import abi_call as _abi_call, module_call as _module_call
 
 pytestmark = pytest.mark.gpu
 
@@ -95,30 +95,6 @@ def qc():
 def ref():
     """Outputs of the reference's kernels: {"matvec": npz, "batched": npz}."""
     return {k: np.load(os.path.join(GOLDEN, f"refparity_{k}.npz")) for k in ("matvec", "batched")}
-
-
-def _abi_call(lib, T, x, mul, batch=1):
-    a = Args(bits=T["bits"], in_features=T["infeatures"], out_features=T["outfeatures"], batch=batch,
-             qweight=T["qweight"].data_ptr(), lookup_table=T["lookup_table"].data_ptr(), vec=x.data_ptr(), mul=mul.data_ptr())
-    if T["rows"] is not None:
-        a.rows, a.cols, a.vals = T["rows"].data_ptr(), T["cols"].data_ptr(), T["vals"].data_ptr()
-    if T["full_rows"] is not None:
-        a.full_rows, a.full_row_indices, a.topX = T["full_rows"].data_ptr(), T["full_row_indices"].data_ptr(), T["full_rows"].shape[1]
-    rc = lib.sqllm_lutgemv(ctypes.byref(a), ctypes.c_void_p(torch.cuda.current_stream().cuda_stream))
-    assert rc == 0, lib.sqllm_last_error()
-
-
-def _module_call(mod, T, x, mul, batched):
-    """The way squeezellm/quant.py:225-309 / :323-379 picks one of the 12 symbols."""
-    b, sfx = T["bits"], "_batched" if batched else ""
-    if T["rows"] is not None and T["full_rows"] is not None:
-        getattr(mod, f"vecquant{b}matmul_spmv_hybrid_nuq_perchannel{sfx}")(
-            T["rows"], T["cols"], T["vals"], x, T["full_rows"], T["full_row_indices"], mul, T["outfeatures"], T["qweight"], T["lookup_table"])
-    elif T["rows"] is not None:
-        getattr(mod, f"vecquant{b}matmul_spmv_nuq_perchannel{sfx}")(
-            T["rows"], T["cols"], T["vals"], x, mul, T["outfeatures"], T["qweight"], T["lookup_table"])
-    else:
-        getattr(mod, f"vecquant{b}matmul_nuq_perchannel{sfx}")(x, T["qweight"], mul, T["lookup_table"])
 
 
 @pytest.mark.parametrize("bits", [3, 4])

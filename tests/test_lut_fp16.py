@@ -35,6 +35,8 @@ SHAPES = [  # (bits, K, N, sparsity, topX, nonzero_full_rows, skew)
     (3, 8192, 22016, 0.0045, 10, False, False),
     (3, 22016, 8192, 0.0045, 10, False, False),
     (3, 8192, 2752, 0.0045, 10, False, False),
+    (4, 4096, 4096, 0.0045, 64, True, False),   # > 32 dense rows: the finisher's general dense-row path
+    (3, 512, 132, 0.01, 128, True, False),      # MAX_TOPX_FUSED dense rows on a ragged 3-strip layer
 ]
 IDS = [f"w{b}-{k}x{n}-s{int(s*1e4)}-t{t}" for b, k, n, s, t, z, sk in SHAPES]
 NORM_TOL = REL_TOL       # max-norm relative error against the exact-codebook result

@@ -67,10 +67,14 @@ def test_pack_unpack_roundtrip_random_words(bits):
 
 
 @pytest.mark.parametrize("bits,K,N,sp,topx", [(4, 128, 64, 0.0, 0), (3, 128, 64, 0.0, 0), (4, 256, 128, 0.02, 0),
-                                                (3, 256, 128, 0.02, 3), (4, 128, 192, 0.01, 10)])
+                                                (3, 256, 128, 0.02, 3), (4, 128, 192, 0.01, 10), (4, 256, 192, 0.01, 64)])
 def test_oracle_forward_against_plain_numpy(bits, K, N, sp, topx):
     """forward_f64 == dequantise with the (golden-pinned) unpack, then a float64 matmul + dense CSR + dense rows."""
     L = orc.make_layer(bits, K, N, sparsity=sp, topX=topx, seed=11, nonzero_full_rows=True)
+    if topx:  # several dense rows on one output channel: every odd row shares the channel of the row before it, a quarter share channel 0
+        fri = L["full_row_indices"]
+        fri[1::2] = fri[0::2][:len(fri[1::2])]
+        fri[3::4] = 0
     x = orc.make_vec(K, batch=3, seed=5)
     idx = orc.unpack_np(L["qweight"], bits).astype(np.int64)             # [K, N]
     W = np.take_along_axis(L["lookup_table"].astype(np.float64).T, idx, axis=0)  # W[k, c] = LUT[c, idx[k, c]]

@@ -5,7 +5,7 @@ import numpy as np
 import pytest
 import torch
 
-from util import REL_TOL, orc, rel_err
+from util import REL_TOL, oracle_chain as _oracle_chain, orc, rel_err
 
 pytestmark = pytest.mark.gpu
 
@@ -19,34 +19,51 @@ def _module(L, bits, K, N, topX):
     return m.cuda()
 
 
+def _scaled_layer(bits, K, N, sparsity, topX, seed, dup):
+    L = orc.make_layer(bits, K, N, sparsity=sparsity, topX=topX, seed=seed, nonzero_full_rows=True)
+    if topX and sparsity == 0:
+        L["full_rows"] = L["full_row_indices"] = None
+    elif topX >= 3 and dup:  # dense rows that feed the same output channel (their parts travel combined), one of them channel 0
+        L["full_row_indices"][1] = L["full_row_indices"][0]
+        L["full_row_indices"][2] = 0
+    # keep activations O(1) through the chain
+    L["lookup_table"] = (L["lookup_table"] * (50.0 / np.sqrt(K))).astype(np.float32)  # centroids ~ N(0, 1/K): |y| ~ |x|
+    return L
+
+
+def _stack_layers(Ls):
+    """numpy restatement of stacking sibling layers along the output dimension (fusion.stack_buffers), for the oracle."""
+    offs = np.cumsum([0] + [L["outfeatures"] for L in Ls])
+    S = dict(bits=Ls[0]["bits"], infeatures=Ls[0]["infeatures"], outfeatures=int(offs[-1]), bias=None)
+    S["qweight"] = np.concatenate([L["qweight"] for L in Ls], axis=1)
+    S["lookup_table"] = np.concatenate([L["lookup_table"] for L in Ls], axis=0)
+    S["rows"] = np.concatenate([[0]] + [L["rows"][1:] + sum(int(P["rows"][-1]) for P in Ls[:i]) for i, L in enumerate(Ls)]).astype(np.int32)
+    S["cols"] = np.concatenate([L["cols"] for L in Ls])
+    S["vals"] = np.concatenate([L["vals"] for L in Ls])
+    S["full_rows"] = np.concatenate([L["full_rows"] for L in Ls], axis=1)
+    S["full_row_indices"] = np.concatenate([L["full_row_indices"] + o for L, o in zip(Ls, offs)]).astype(np.int32)
+    return S
+
+
 def _chain(bits, dims, sparsity, topX, seed):
-    """dims: [(K, N, x_offset into the previous output)]; returns oracle layers + modules."""
+    """dims: [(K, N, x_offset into the previous output[, members])]; returns oracle layers + modules.  An item with members > 1 is
+    the stacked layer that fusion.fuse_siblings builds from that many sibling layers of N / members columns and topX dense rows each."""
+    from squeezellm_b200.fusion import SiblingGroup
     layers, mods = [], []
-    for i, (K, N, _) in enumerate(dims):
-        L = orc.make_layer(bits, K, N, sparsity=sparsity, topX=topX, seed=seed + 17 * i, nonzero_full_rows=True)
-        if topX and sparsity == 0:
-            L["full_rows"] = L["full_row_indices"] = None
-        elif topX >= 3 and i % 2 == 0:  # dense rows that feed the same output channel (their parts travel combined), one of them channel 0
-            L["full_row_indices"][1] = L["full_row_indices"][0]
-            L["full_row_indices"][2] = 0
-        # keep activations O(1) through the chain
-        L["lookup_table"] = (L["lookup_table"] * (50.0 / np.sqrt(K))).astype(np.float32)  # centroids ~ N(0, 1/K): |y| ~ |x|
+    for i, d in enumerate(dims):
+        K, N = d[0], d[1]
+        members = d[3] if len(d) > 3 else 1
+        if members == 1:
+            L = _scaled_layer(bits, K, N, sparsity, topX, seed + 17 * i, dup=i % 2 == 0)
+            m = _module(L, bits, K, N, topX)
+        else:
+            Ls = [_scaled_layer(bits, K, N // members, sparsity, topX, seed + 17 * i + 1000 * j, dup=j == 0) for j in range(members)]
+            L = _stack_layers(Ls)
+            m = SiblingGroup([_module(Lj, bits, K, N // members, topX) for Lj in Ls]).layer
+            assert m.topX == members * topX
         layers.append(L)
-        mods.append(_module(L, bits, K, N, topX))
+        mods.append(m)
     return layers, mods
-
-
-def _oracle_chain(layers, dims, x, lut_fp16=False):
-    outs, prev = [], None
-    for L, (K, N, off) in zip(layers, dims):
-        xin = x if prev is None else prev[off:off + K]
-        LL = dict(L)
-        if lut_fp16:
-            LL["lookup_table"] = L["lookup_table"].astype(np.float16).astype(np.float32)
-        y = orc.forward_f64(LL, xin.astype(np.float32).reshape(1, K)).reshape(N)
-        prev = y.astype(np.float16).astype(np.float64)  # the hand-over between two matvecs is fp16, as in the model
-        outs.append(prev)
-    return outs
 
 
 CASES = [  # (bits, dims, sparsity, topX)
@@ -56,8 +73,10 @@ CASES = [  # (bits, dims, sparsity, topX)
     (4, [(512, 132, 0), (128, 200, 4), (192, 64, 8), (64, 512, 0), (512, 132, 0)], 0.01, 3),   # ragged strips, one-strip items
     (4, [(4096, 12288, 0), (4096, 4096, 8192), (4096, 22016, 0), (11008, 4096, 0)], 0.0045, 10, 3),  # LLaMA-7B decoder layer, three times over
     (3, [(4096, 12288, 0), (4096, 4096, 8192), (4096, 22016, 0), (11008, 4096, 0)], 0.0045, 10, 2),
+    (4, [(256, 768, 0), (256, 256, 512), (256, 704, 0), (704, 256, 0)], 0.02, 43),        # > 32 dense rows per item, duplicate channels
+    (4, [(512, 768, 0, 3), (256, 256, 512), (256, 768, 0, 3), (768, 132, 0)], 0.02, 11),  # stacked q+k+v of topX = 11: 33 dense rows
 ]
-IDS = [f"w{c[0]}-{len(c[1])}items-K{c[1][0][0]}-s{int(c[2] * 1e4)}-t{c[3]}" for c in CASES]
+IDS = [f"w{c[0]}-{len(c[1])}items-K{c[1][0][0]}-s{int(c[2] * 1e4)}-t{c[3]}{'-stacked' if len(c[1][0]) > 3 else ''}" for c in CASES]
 
 
 @pytest.mark.parametrize("case", CASES, ids=IDS)
@@ -72,6 +91,7 @@ def test_sequence_matches_layer_by_layer_and_oracle(case, mode):
     x = orc.make_vec(dims[0][0], seed=5).reshape(-1).astype(np.float16)
     seq = DecodeSequence(dims[0][0], "cuda", lut_mode=mode)
     vecs, prev = [], seq.input
+    dims = [d[:3] for d in dims]
     for m, (K, N, off) in zip(mods, dims):
         prev = seq.matvec(m, prev[off:off + K])
         vecs.append(prev)

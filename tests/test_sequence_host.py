@@ -68,3 +68,16 @@ def test_create_rejects_bad_arguments(items, kw, needle):
     lib = load_lib()
     rc, msg = _create(lib, items, **kw) if items else (lib.sqllm_sequence_create(None, 0, None, None), lib.sqllm_last_error().decode())
     assert rc == -1 and needle in msg, (rc, msg)
+
+
+@pytest.mark.parametrize("topX,N,needle", [(129, 128, "MAX_TOPX_FUSED"), (10, 262148, "MAX_N_FUSED")])
+def test_matvec_rejects_layers_past_the_fused_limits(topX, N, needle):
+    """DecodeSequence.matvec refuses, when the layer is recorded, what the sequence kernel cannot run (not later, inside compile)."""
+    from squeezellm_b200.quant import QuantLinearLUT, quant_cuda
+    from squeezellm_b200.runtime import DecodeSequence
+    assert (quant_cuda.MAX_TOPX_FUSED, quant_cuda.MAX_N_FUSED) == (128, 262144)
+    seq = DecodeSequence(64, "cpu")
+    ok = QuantLinearLUT(4, 64, 128, False, include_sparse=True, numvals=1, topX=quant_cuda.MAX_TOPX_FUSED)
+    seq.matvec(ok, seq.input)
+    with pytest.raises(ValueError, match=needle):
+        seq.matvec(QuantLinearLUT(4, 64, N, False, include_sparse=True, numvals=1, topX=topX), seq.input)

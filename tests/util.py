@@ -69,3 +69,44 @@ def to_torch(layer, device="cuda"):
     for k, v in layer.items():
         out[k] = torch.from_numpy(v).to(device) if isinstance(v, np.ndarray) else v
     return out
+
+
+def abi_call(lib, T, x, mul, batch=1):
+    """sqllm_lutgemv (accumulate into mul) on the current stream for the torch layer T (to_torch)."""
+    import torch
+    a = Args(bits=T["bits"], in_features=T["infeatures"], out_features=T["outfeatures"], batch=batch,
+             qweight=T["qweight"].data_ptr(), lookup_table=T["lookup_table"].data_ptr(), vec=x.data_ptr(), mul=mul.data_ptr())
+    if T["rows"] is not None:
+        a.rows, a.cols, a.vals = T["rows"].data_ptr(), T["cols"].data_ptr(), T["vals"].data_ptr()
+    if T["full_rows"] is not None:
+        a.full_rows, a.full_row_indices, a.topX = T["full_rows"].data_ptr(), T["full_row_indices"].data_ptr(), T["full_rows"].shape[1]
+    rc = lib.sqllm_lutgemv(ctypes.byref(a), ctypes.c_void_p(torch.cuda.current_stream().cuda_stream))
+    assert rc == 0, lib.sqllm_last_error()
+
+
+def module_call(mod, T, x, mul, batched):
+    """The way squeezellm/quant.py:225-309 / :323-379 picks one of the 12 symbols."""
+    b, sfx = T["bits"], "_batched" if batched else ""
+    if T["rows"] is not None and T["full_rows"] is not None:
+        getattr(mod, f"vecquant{b}matmul_spmv_hybrid_nuq_perchannel{sfx}")(
+            T["rows"], T["cols"], T["vals"], x, T["full_rows"], T["full_row_indices"], mul, T["outfeatures"], T["qweight"], T["lookup_table"])
+    elif T["rows"] is not None:
+        getattr(mod, f"vecquant{b}matmul_spmv_nuq_perchannel{sfx}")(
+            T["rows"], T["cols"], T["vals"], x, mul, T["outfeatures"], T["qweight"], T["lookup_table"])
+    else:
+        getattr(mod, f"vecquant{b}matmul_nuq_perchannel{sfx}")(x, T["qweight"], mul, T["lookup_table"])
+
+
+def oracle_chain(layers, dims, x, lut_fp16=False):
+    """fp64 truth of a chain of matvecs, dims = [(K, N, x_offset into the previous output), ...]; the hand-over between two
+    matvecs is rounded to fp16, as in the model (and in the sequence kernel)."""
+    outs, prev = [], None
+    for L, (K, N, off) in zip(layers, dims):
+        xin = x if prev is None else prev[off:off + K]
+        LL = dict(L)
+        if lut_fp16:
+            LL["lookup_table"] = L["lookup_table"].astype(np.float16).astype(np.float32)
+        y = orc.forward_f64(LL, xin.astype(np.float32).reshape(1, K)).reshape(N)
+        prev = y.astype(np.float16).astype(np.float64)
+        outs.append(prev)
+    return outs
